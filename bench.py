@@ -2,6 +2,7 @@
 """bench.py — throughput of the fused score -> top-k -> gather path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--no-extras]
+                    [--dump-outputs DIR]
 
 A "step" is one ScorerPress.compress call on one layer's synthetic cache [B, Hkv, S, D] (bf16).
 Prints ONE JSON line on rank 0:
@@ -426,18 +427,48 @@ def bind_to_gpu_numa(local_rank: int):
 
 def timed_loop(calls, steps: int):
     """`steps` back-to-back calls (calls[i % len]) bracketed by CUDA events on the current stream. Returns
-    (device ms per step, host us per call spent enqueueing)."""
+    (device ms per step, host us per call spent enqueueing, what the last call returned)."""
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     n = len(calls)
+    last = None
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     start.record()
     for i in range(steps):
-        calls[i % n]()
+        last = calls[i % n]()
     stop.record()
     host_us = (time.perf_counter() - t0) / steps * 1e6
     torch.cuda.synchronize()
-    return start.elapsed_time(stop) / steps, host_us
+    return start.elapsed_time(stop) / steps, host_us, last
+
+
+DUMP_BUDGET_BYTES = 60 << 20      # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir: str, w: dict, outputs) -> dict:
+    """Writes what one timed call returned as <out_dir>/<name>.npy: the compacted keys / values as float32, or (AdaKV)
+    the pruned flat indices as float64, which holds them exactly. An array above its share of DUMP_BUDGET_BYTES is cut
+    to a fixed sample of its rows (last axis kept whole): the first rows of a seeded permutation, in ascending order,
+    so that two builds given the same arguments write the same rows. Returns {name: what was written}."""
+    import numpy as np
+
+    names = ("pruned_indices",) if w["scorer"] == "adakv_ea" else ("keys", "values")
+    arrays = {n: t for n, t in zip(names, outputs) if t is not None}
+    budget = DUMP_BUDGET_BYTES // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    written = {}
+    for name, t in arrays.items():
+        t = t.detach().to("cpu", torch.float64 if name == "pruned_indices" else torch.float32)
+        rows = t.reshape(-1, t.shape[-1])
+        n_rows = max(1, budget // (rows.shape[1] * rows.element_size()))
+        sampled = n_rows < rows.shape[0]
+        if sampled:
+            pick = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:n_rows].sort().values
+            t = rows[pick]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
+        written[name] = {"shape": list(t.shape), "dtype": str(t.dtype).replace("torch.", ""),
+                         "sampled_rows_of": list(rows.shape) if sampled else None}
+    return written
 
 
 # --------------------------------------------------------------------------------------------------
@@ -455,10 +486,10 @@ def extra_workload(name: str, device, rank: int, steps: int, peaks: dict) -> dic
     graphs = [native.capture(lambda s=s: run_native(w, s[0], s[1], s[2], n_kept)) for s in sets]
     calls = [g.replay for g in graphs]
     timed_loop(calls, 3)
-    ms, host_us = timed_loop(calls, steps)
+    ms, host_us, _ = timed_loop(calls, steps)
     eager = [lambda s=s: run_native(w, s[0], s[1], s[2], n_kept) for s in sets]
     timed_loop(eager, 3)
-    ms_e, host_e = timed_loop(eager, steps)
+    ms_e, host_e, _ = timed_loop(eager, steps)
     abytes = algorithmic_bytes(w, n_kept)
     out = {"workload": name, "baseline_config_index": w["config_index"], "description": w["label"],
            "us_per_step": ms * 1e3, "tokens_per_s": w["B"] * w["S"] / (ms * 1e-3), "steps": steps,
@@ -504,7 +535,7 @@ def extra_layer_split(device, rank: int, world: int, dist, steps: int, n_layers:
     for _ in range(2):
         call()
     barrier()
-    ms, host_us = timed_loop([call], steps)
+    ms, host_us, _ = timed_loop([call], steps)
     barrier()
     ms = max_over_ranks(ms, dist, device)
     abytes = algorithmic_bytes(w, n_kept) * len(mine)
@@ -658,7 +689,13 @@ def main():
     ap.add_argument("--cpu-step-budget", type=float, default=None,
                     help="seconds one CPU call of the reference arm may take (sizes its bounded sample); default: "
                          "chosen so that warmup + steps calls end within ~2 minutes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32 / "
+                         "float64, under 64 MB in all: larger outputs as a fixed seeded sample of rows); with the same "
+                         "arguments the inputs are the same on every run, so two builds can be compared output by output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", 0))
@@ -733,12 +770,15 @@ def main():
     calls = [g.replay for g in graphs] if graphs is not None else eager_calls
     barrier()
     with ClockSampler(local_rank) as clocks:
-        ms_local, host_us = timed_loop(calls, args.steps)
+        ms_local, host_us, last_out = timed_loop(calls, args.steps)
     barrier()
     ms_per_step = max_over_ranks(ms_local, dist, device)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = {"dir": args.dump_outputs, "arrays": dump_outputs(args.dump_outputs, w, last_out)}
     eager = None
     if graphs is not None:
-        ms_e, host_e = timed_loop(eager_calls, args.steps)
+        ms_e, host_e, _ = timed_loop(eager_calls, args.steps)
         barrier()
         eager = {"ms_per_step": max_over_ranks(ms_e, dist, device), "host_us_per_call": host_e}
     tokens_per_step = w["B"] * w["S"] * world
@@ -888,6 +928,8 @@ def main():
         "clocks": clocks.summary(), "token_heads_per_s": value * w["Hkv"],
         "extras": extras, "extras_errors": extras_errors,
     }
+    if dumped is not None:
+        line["dumped_outputs"] = dumped
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

@@ -11,6 +11,7 @@ Run in the build container, where /root/reference exists:  python oracle/build_r
 """
 from __future__ import annotations
 
+import os
 import shutil
 import sys
 from pathlib import Path
@@ -24,7 +25,7 @@ def build_ref(force: bool = False) -> Path | None:
     marker = DEST / "kvpress" / "__init__.py"
     if marker.exists() and not force:
         return DEST
-    if not (REFERENCE / "kvpress" / "__init__.py").exists():
+    if not os.path.isfile(REFERENCE / "kvpress" / "__init__.py"):     # absent, or not readable by this user
         return DEST if marker.exists() else None
     if DEST.exists():
         shutil.rmtree(DEST)

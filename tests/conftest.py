@@ -1,3 +1,4 @@
+import os
 import sys
 from pathlib import Path
 
@@ -60,7 +61,7 @@ def golden_or_live(request) -> Golden:
     """The stored cases plus, where the reference is importable, the same cases generated live on this host."""
     name = request.param
     if name.startswith("live:"):
-        if not REFERENCE_DIR.exists():
+        if not os.path.isdir(REFERENCE_DIR):             # absent, or not readable by this user
             pytest.skip("no /root/reference here: live pinning runs in the build container only")
         return Golden(name[5:], live=True)
     return Golden(name)

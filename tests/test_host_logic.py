@@ -30,7 +30,8 @@ def model():
 
 @pytest.fixture(scope="module")
 def pipe():
-    return KVPressTextGenerationPipeline(model=tiny_llama(), tokenizer=word_tokenizer())
+    # device pinned: with a GPU present, transformers' Pipeline would move the CPU model to cuda:0
+    return KVPressTextGenerationPipeline(model=tiny_llama(), tokenizer=word_tokenizer(), device="cpu")
 
 
 def test_product_refuses_cpu_tensors_without_backend():
