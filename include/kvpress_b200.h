@@ -98,7 +98,7 @@ const char* kvp_last_cuda_error(void);
 /* Bytes of scratch a *_compress / *_score call of this scorer needs (256-byte aligned). */
 int kvp_workspace_bytes(const kvp_problem* p, int scorer, size_t* bytes_out);
 
-/* Debugging aid. The persistent select / compact kernels wait on each other with BOUNDED spins; a wait that
+/* Debugging aid. The work items of the persistent Knorm kernel wait on each other with BOUNDED spins; a wait that
  * expires raises a flag in the workspace instead of trapping the CUDA context. This call synchronises
  * `stream`, reads the flag of the last call that used `workspace` and returns KVP_OK or
  * KVP_ERR_KERNEL_TIMEOUT. Never needed for correct operation. */

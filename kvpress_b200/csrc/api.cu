@@ -22,14 +22,22 @@ static int fail_cuda(cudaError_t e) {
 
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-static int validate(const kvp_problem* p, Dims* d, bool need_kv_strides = true) {
+// Rows (B * Hkv) a call may have. The score kernels put the row on gridDim.y (<= 65535). The generic-score path
+// (keys_from_scores + selection pass + compaction grid) decodes rows from a 1-D grid of rows x tiles, which only
+// needs that product to fit an int; the row cap keeps the counter slots (3 R + 8) in range.
+constexpr int64_t kMaxRowsGridY = 65535;
+constexpr int64_t kMaxRowsGeneric = (int64_t)1 << 24;
+static int64_t max_rows(int scorer) { return scorer == KVP_SCORER_GENERIC ? kMaxRowsGeneric : kMaxRowsGridY; }
+
+static int validate(const kvp_problem* p, Dims* d, bool need_kv_strides = true, int64_t row_cap = kMaxRowsGridY) {
     if (p == nullptr) return KVP_ERR_NULL_POINTER;
     if (p->dtype != KVP_BF16 && p->dtype != KVP_F16) return KVP_ERR_UNSUPPORTED_DTYPE;
     if (p->B <= 0 || p->Hkv <= 0 || p->S <= 0 || p->D <= 0) return KVP_ERR_UNSUPPORTED_SHAPE;
     if (p->D % 8 != 0 || p->D > 256) return KVP_ERR_UNSUPPORTED_SHAPE;
     if (p->Hq <= 0 || p->Hq % p->Hkv != 0) return KVP_ERR_UNSUPPORTED_SHAPE;
     if (p->n_kept < 0 || p->n_kept > p->S) return KVP_ERR_BAD_ARGUMENT;
-    if ((int64_t)p->B * p->Hkv > 65535) return KVP_ERR_UNSUPPORTED_SHAPE;  // gridDim.y
+    if ((int64_t)p->B * p->Hkv > row_cap) return KVP_ERR_UNSUPPORTED_SHAPE;
+    if ((int64_t)p->B * p->Hkv * ((p->S + kTile - 1) / kTile) > 0x7FFFFFFF) return KVP_ERR_UNSUPPORTED_SHAPE;  // 1-D grids
     if (need_kv_strides) {
         for (int i = 0; i < 3; ++i) {
             // rows must stay 16-byte aligned: every outer stride is a multiple of 8 elements
@@ -142,7 +150,7 @@ const char* kvp_last_cuda_error(void) { return g_last_cuda_error; }
 
 int kvp_workspace_bytes(const kvp_problem* p, int scorer, size_t* bytes_out) {
     Dims d;
-    int rc = validate(p, &d, false);
+    int rc = validate(p, &d, false, max_rows(scorer));
     if (rc) return rc;
     if (!bytes_out) return KVP_ERR_NULL_POINTER;
     // window only changes the SnapKV scratch; size for the largest supported window
@@ -153,7 +161,7 @@ int kvp_workspace_bytes(const kvp_problem* p, int scorer, size_t* bytes_out) {
 int kvp_workspace_check(const kvp_problem* p, int scorer, const void* workspace, size_t workspace_bytes,
                         kvp_stream_t stream) {
     Dims d;
-    int rc = validate(p, &d, false);
+    int rc = validate(p, &d, false, max_rows(scorer));
     if (rc) return rc;
     Workspace ws;
     WsLayout L;
@@ -171,20 +179,21 @@ int kvp_launches_per_compress(const kvp_problem* p, int scorer, int* launches_ou
     if (!p || !launches_out) return KVP_ERR_NULL_POINTER;
     switch (scorer) {
         case KVP_SCORER_STREAMING: *launches_out = 1; break;
-        case KVP_SCORER_GENERIC: *launches_out = 3; break;  // memset, keys, select+compact
-        case KVP_SCORER_KNORM: {  // cluster kernel | memset + (fused | score, select+compact)
+        // "select, compact" below: the selection pass and the compaction grid (select_compact.cu)
+        case KVP_SCORER_GENERIC: *launches_out = 4; break;  // memset, keys, select, compact
+        case KVP_SCORER_KNORM: {  // cluster kernel | memset + (fused | score, select, compact)
             Dims d;
             if (validate(p, &d, false) == KVP_OK && knorm_cluster_applicable(d)) *launches_out = 1;
-            else *launches_out = ((size_t)p->B * p->Hkv * p->S * p->D * 2 <= ((size_t)32 << 20)) ? 2 : 3;
+            else *launches_out = ((size_t)p->B * p->Hkv * p->S * p->D * 2 <= ((size_t)32 << 20)) ? 2 : 4;
             break;
         }
-        case KVP_SCORER_KEYDIFF: *launches_out = 5; break;  // memset, anchor partials, merge, score, select+compact
-        case KVP_SCORER_SNAPKV: *launches_out = 6; break;  // memset, stats, memset, colsum, finalize, select+compact
+        case KVP_SCORER_KEYDIFF: *launches_out = 6; break;  // memset, anchor partials, merge, score, select, compact
+        case KVP_SCORER_SNAPKV: *launches_out = 7; break;  // memset, stats, memset, colsum, finalize, select, compact
         case KVP_SCORER_EXPECTED_ATTENTION: {
             // press defaults (use_covariance + use_vnorm): memset, logits (the tensor-core kernels stage the V tiles and
-            // take the value norms themselves), finalize, select+compact; head dims outside 64 / 128 have no covariance
+            // take the value norms themselves), finalize, select, compact; head dims outside 64 / 128 have no covariance
             // path here, and the covariance-free scan adds the value-norm kernel on the side stream
-            *launches_out = (p->D == 64 || p->D == 128) ? 4 : 5;
+            *launches_out = (p->D == 64 || p->D == 128) ? 5 : 6;
             break;
         }
         default: return KVP_ERR_BAD_ARGUMENT;
@@ -412,7 +421,7 @@ int kvp_scores_compress(const kvp_problem* p, const void* scores, const int64_t*
                         int32_t* idx_out, void* workspace, size_t workspace_bytes,
                         kvp_stream_t stream) {
     Dims d;
-    int rc = validate(p, &d);
+    int rc = validate(p, &d, true, kMaxRowsGeneric);
     if (rc) return rc;
     if (d.n_kept == 0) return KVP_OK;
     if ((rc = check_io(K, V, K_out, V_out))) return rc;
@@ -431,7 +440,7 @@ int kvp_scores_compress(const kvp_problem* p, const void* scores, const int64_t*
 int kvp_scores_select(const kvp_problem* p, const void* scores, const int64_t* score_stride,
                       int32_t* idx_out, void* workspace, size_t workspace_bytes, kvp_stream_t stream) {
     Dims d;
-    int rc = validate(p, &d, false);
+    int rc = validate(p, &d, false, kMaxRowsGeneric);
     if (rc) return rc;
     if (d.n_kept == 0) return KVP_OK;
     if (!scores || !score_stride || !idx_out) return KVP_ERR_NULL_POINTER;
@@ -452,7 +461,7 @@ int kvp_scores_compress_rerotate(const kvp_problem* p, const void* scores, const
                                  void* V_out, int32_t* idx_out, void* workspace,
                                  size_t workspace_bytes, kvp_stream_t stream) {
     Dims d;
-    int rc = validate(p, &d);
+    int rc = validate(p, &d, true, kMaxRowsGeneric);
     if (rc) return rc;
     if (d.D % 16 != 0) return KVP_ERR_UNSUPPORTED_SHAPE;  // rotate_half pairs d with d + D/2
     if (d.n_kept == 0) return KVP_OK;

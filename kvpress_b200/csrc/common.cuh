@@ -17,7 +17,7 @@ constexpr int kSfxStride = 264;     // u16 per tile record: sfx[0..256], gt_hi a
 constexpr uint16_t kForcedKey = 0xFFFFu;  // ordered key of a forced-keep position
 constexpr int kFinalizeTiles = 1;          // 256-position tiles per CTA of the finalize kernels (1: >5 waves at 128k, no tail)
 constexpr int kScoreChunkGeneric = 256;   // positions per CTA of the plain streaming score kernels
-// counters[] layout: [0] ticket, [1, 1+R) refine done, [1+R, 1+2R) row ready, then the slot below:
+// counters[] layout: [0] ticket (fused Knorm kernel), [1, 1+R) refine done, [1+R, 1+2R) row ready, then the slot below:
 // order-preserving uint image of the largest valid score (for the reference's max+1 sentinel);
 // [2+2R, 2+3R) score items done per row (fused Knorm kernel)
 __host__ __device__ constexpr int kCounterMaxSlot(int R) { return 1 + 2 * R; }
@@ -133,10 +133,10 @@ __device__ __forceinline__ void stg_hint(void* p, const int4& v, uint64_t pol) {
 }
 
 // ---- programmatic dependent launch (PDL) ------------------------------------------------------------------
-// The select+compact kernel is launched with cudaLaunchAttributeProgrammaticStreamSerialization: its CTAs may
-// become resident while the LAST wave of the score / finalize kernel in front of it is still draining (that kernel
+// The selection pass and the compaction grid are launched with cudaLaunchAttributeProgrammaticStreamSerialization:
+// their CTAs may become resident while the LAST wave of the kernel in front of them is still draining (that kernel
 // calls pdl_launch_dependents() at its start) and park in pdl_wait() until that grid has completed and flushed, so
-// the launch latency and the ramp of the persistent grid are off the critical path. Both are no-ops for a plain launch.
+// the launch latency and the ramp of each grid are off the critical path. Both are no-ops for a plain launch.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 

@@ -1144,7 +1144,7 @@ ea_finalize_kernel(int G, int S, int n_sink, int use_vnorm, float eps, int n_par
     __shared__ float s_max[8];
     const int chunk = blockIdx.x, row = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     shist[tid] = 0;
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     const int s0 = chunk * kEaFinalPos + tid * KPT;
     const bool in_pad = s0 < ws.S_pad;  // the padded scratch rows are readable up to S_pad (a multiple of 256)
     // 1. independent loads first: this thread's logits / norms and (warps < G) the per-CTA softmax partials
@@ -1235,7 +1235,7 @@ template <typename T>
 __global__ void fill_sentinel_kernel(uint16_t* __restrict__ scores_out, int R, int S, int lo, int hi,
                                      const uint32_t* __restrict__ max_slot) {
     const uint32_t ord = *max_slot;
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     const uint32_t u = (ord & 0x80000000u) ? (ord & 0x7FFFFFFFu) : ~ord;
     const float sentinel = __uint_as_float(u) + 1.0f;
     const uint16_t bits = F16Traits<T>::from_float(sentinel);

@@ -169,7 +169,7 @@ keydiff_score_kernel(const T* __restrict__ K, Strides3 ks, int H, int S, int D, 
     const int b = row / H, h = row % H;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     shist[tid] = 0;
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     constexpr int RPW = 32 / LPR;
     constexpr int TOK_PER_WARP = kScoreChunk / (kTileThreads / 32);
     constexpr int ITERS = TOK_PER_WARP / RPW;

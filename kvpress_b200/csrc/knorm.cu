@@ -22,7 +22,7 @@ knorm_score_kernel(const T* __restrict__ K, Strides3 ks, int H, int S, int D, Wo
     __shared__ uint32_t shist[256];
     const int chunk = blockIdx.x, row = blockIdx.y, tid = threadIdx.x;
     shist[tid] = 0;  // kTileThreads == 256
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     // L2 plan of a compress call (keep_from_row >= 0): the compaction stage re-reads the kept K rows, last rows first.
     // The rows it reaches while they can still be in L2 are loaded evict_last, the earlier ones evict_first, so that
     // the stream of early rows does not push the late ones out (profiles/r02_ab_knorm_l2.txt).
@@ -81,10 +81,13 @@ keys_from_scores_kernel(const uint16_t* __restrict__ scores, int64_t sb, int64_t
                         uint16_t inf_bits, Workspace ws) {
     __shared__ uint16_t skeys[kTile];
     __shared__ uint32_t shist[256];
-    const int tile = blockIdx.x, row = blockIdx.y, tid = threadIdx.x;
+    // 1-D grid of rows x tiles: the generic-score path accepts more than 65535 rows (gridDim.y)
+    const int n_tiles = ws.n_tiles;
+    const int tile = (int)(blockIdx.x % (unsigned)n_tiles), row = (int)(blockIdx.x / (unsigned)n_tiles);
+    const int tid = threadIdx.x;
     const int b = row / H, h = row % H;
     shist[tid] = 0;
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     const uint16_t* src = scores + (int64_t)b * sb + (int64_t)h * sh;
     const int s = tile * kTile + tid;
     skeys[tid] = (s < S) ? ordered_key16(src[s], inf_bits) : (uint16_t)0;
@@ -94,8 +97,7 @@ keys_from_scores_kernel(const uint16_t* __restrict__ scores, int64_t sb, int64_t
 
 cudaError_t launch_keys_from_scores(const Dims& d, int dtype, const void* scores, int64_t sb, int64_t sh,
                                     const Workspace& ws, cudaStream_t st) {
-    const int n_tiles = (d.S + kTile - 1) / kTile;
-    dim3 grid(n_tiles, d.R);
+    const dim3 grid(d.R * ws.n_tiles);
     keys_from_scores_kernel<<<grid, kTileThreads, 0, st>>>(static_cast<const uint16_t*>(scores),
                                                            sb, sh, d.H, d.S,
                                                            dtype == KVP_BF16 ? 0x7F80u : 0x7C00u, ws);

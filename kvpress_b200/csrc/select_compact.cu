@@ -3,16 +3,18 @@
 // Replaces scores.topk(n_kept).indices + keys.gather + values.gather
 // (kvpress/presses/scorer_press.py:95-100) for 16-bit scores:
 //   * the score stage left, per (b,h) row, the ordered keys and a 256-bin histogram of key>>8;
-// ONE persistent kernel (select_compact_kernel) pulls two kinds of items from a ticket counter:
-//   * refine item  : (row, 8 tiles) finds the threshold bin b1 from that histogram, histograms the
-//                    low byte of the keys that fall in b1 (-> row hist_lo, one warp per tile) and
-//                    records, per tile, the suffix counts of those low bytes + the count of keys
-//                    above b1; then bumps the row's "refined" counter;
-//   * compact item : (row, tile) waits for the row's counter, derives the exact 16-bit threshold T
-//                    and the number of ties to take, sums the records of the tiles before it, ranks
-//                    its own 1024 positions with one block scan and copies the kept K and V rows
-//                    (16-byte vectors, 8 in flight per thread) to [B,H,n_kept,D] in ascending
-//                    position order. Ties at T go to the lowest positions.
+// Two kernels, chained by programmatic dependent launch (PDL):
+//   * selection pass (select_kernel), one CTA per refine item (row, 16 tiles): finds the threshold
+//                    bin b1 from that histogram, histograms the low byte of the keys that fall in b1
+//                    (-> row hist_lo, one warp per tile) and records, per tile, the suffix counts of
+//                    those low bytes + the count of keys above b1. The CTA that finishes a row's last
+//                    item runs the row scan: exact 16-bit threshold T, number of ties to take, and
+//                    per tile the kept / tied positions of the tiles before it. Nothing in it waits.
+//   * compaction grid (compact_kernel), one CTA per (row, tile of 256 positions): loads its keys,
+//                    its tile prefix and the row's threshold (all final once the selection pass has
+//                    completed), ranks its positions with warp ballots and copies the kept K and V
+//                    rows (16-byte vectors) to [B,H,n_kept,D] in ascending position order. Ties at T
+//                    go to the lowest positions. No waits of any kind.
 // Tiles are visited in REVERSE order of the score stage so the K rows touched last (still in the
 // 126 MB L2) are re-read first.
 #include <stdlib.h>
@@ -23,40 +25,16 @@
 
 namespace kvp {
 
-#ifdef KVP_SEL_PROFILE
-__device__ long long g_sel_prof[16];
-#define SEL_T0(name) const long long name = clock64()
-#define SEL_ACC(slot, name) do { if (blockIdx.x == 0 && threadIdx.x == 0) g_sel_prof[slot] += clock64() - name; } while (0)
-#define SEL_CNT(slot) do { if (blockIdx.x == 0 && threadIdx.x == 0) g_sel_prof[slot] += 1; } while (0)
-extern "C" void kvp_debug_sel_profile(long long* out, int reset) {
-    if (reset) {
-        long long z[16] = {0};
-        cudaMemcpyToSymbol(g_sel_prof, z, sizeof(z));
-    } else {
-        cudaMemcpyFromSymbol(out, g_sel_prof, 16 * sizeof(long long));
-    }
-}
-#else
-#define SEL_T0(name) do {} while (0)
-#define SEL_ACC(slot, name) do {} while (0)
-#define SEL_CNT(slot) do {} while (0)
-#endif
-
-// tuning knobs of the compact items (A/B-tested on the B200, see profiles/)
-#ifndef KVP_SEL_U
-#define KVP_SEL_U 3
-#define KVP_SEL_TWO true
-#define KVP_SEL_CTAS 3
-#endif
-
 constexpr int kTilesPerWarp = 2;                                  // refine: tiles per warp
 constexpr int kGroupTiles = (kTileThreads / 32) * kTilesPerWarp;  // tiles per refine item (16)
+constexpr int kScanTiles = 4;                                     // row scan: consecutive tiles per thread and pass
 
 // Copies `count` rows of `nvec` 16-byte vectors of BOTH tensors: dst row j <- src row list[j].
 // K rows are plain loads (they may still sit in L2 from the score stage), V rows and all stores are
 // streamed (evict-first). The loads of two consecutive batches (2 x 2*U 16-byte loads per thread) are
-// issued before the first store, so a typical item (<= 128 kept rows of 256 B) is ONE memory round trip.
-template <int U, bool kTwoBatches>
+// issued before the first store, so a typical tile (<= 128 kept rows of 256 B) is ONE memory round trip.
+// Generic loads on purpose: host_staging's zero-copy mode gathers V rows from pinned host memory here.
+template <int U>
 __device__ __forceinline__ void copy_rows_kv(const char* __restrict__ srcK, int64_t k_row_bytes,
                                              const char* __restrict__ srcV, int64_t v_row_bytes,
                                              char* __restrict__ dstK, char* __restrict__ dstV,
@@ -90,21 +68,13 @@ __device__ __forceinline__ void copy_rows_kv(const char* __restrict__ srcK, int6
             }
         }
     };
-    if (kTwoBatches) {
-        for (int base = threadIdx.x; base < total; base += 2 * STEP) {
-            int4 ak[U], av[U], bk[U], bv[U];
-            load(ak, av, base);
-            const bool second = (base + STEP) < total;
-            if (second) load(bk, bv, base + STEP);
-            store(ak, av, base);
-            if (second) store(bk, bv, base + STEP);
-        }
-    } else {
-        for (int base = threadIdx.x; base < total; base += STEP) {
-            int4 ak[U], av[U];
-            load(ak, av, base);
-            store(ak, av, base);
-        }
+    for (int base = threadIdx.x; base < total; base += 2 * STEP) {
+        int4 ak[U], av[U], bk[U], bv[U];
+        load(ak, av, base);
+        const bool second = (base + STEP) < total;
+        if (second) load(bk, bv, base + STEP);
+        store(ak, av, base);
+        if (second) store(bk, bv, base + STEP);
     }
 }
 
@@ -175,7 +145,7 @@ struct SelectSmem {
     int list[kTile];
     uint32_t wsum[2][8];
     uint32_t thr[3];
-    uint32_t meta[2];  // compact item: the row's threshold key and tie budget, fetched by the polling thread
+    uint32_t meta[2];  // fused compact item: the row's threshold key and tie budget, fetched by the polling thread
     int item;
     int b1;
     int last;
@@ -205,21 +175,28 @@ __device__ __forceinline__ void scan_row(SelectSmem& sm, int row, int n_kept, co
     __syncthreads();
     const uint32_t lo1 = sm.thr[2];
     if (tid == 0) ws.row_meta[row] = make_uint2(sm.thr[0], sm.thr[1]);
-    __threadfence();  // row_meta is visible before any prefix (= readiness) is
-    __syncthreads();
     const uint16_t* recs = ws.tile_sfx + (size_t)row * ws.n_tiles * kSfxStride;
     uint2* prefix = ws.tile_prefix + (size_t)row * ws.n_tiles;
     uint32_t carry_gt = 0, carry_eq = 0;
-    for (int t0 = 0; t0 < ws.n_tiles; t0 += kTileThreads) {
-        const int t = t0 + tid;
-        uint32_t gt = 0, eq = 0;
-        if (t < ws.n_tiles) {
-            const uint16_t* r = recs + (size_t)t * kSfxStride;
-            const uint32_t ge = __ldcg(r + lo1), g2 = __ldcg(r + lo1 + 1);
-            gt = (uint32_t)__ldcg(r + 257) + g2;
-            eq = ge - g2;
+    // a pass covers kScanTiles consecutive tiles per thread, so tile order == thread order and the records of a
+    // pass are ONE round trip (S <= 256 k: one pass)
+    for (int p0 = 0; p0 < ws.n_tiles; p0 += kScanTiles * kTileThreads) {
+        const int t0 = p0 + tid * kScanTiles;
+        uint32_t gt[kScanTiles], eq[kScanTiles], sum_gt = 0, sum_eq = 0;
+#pragma unroll
+        for (int c = 0; c < kScanTiles; ++c) {
+            gt[c] = eq[c] = 0;
+            if (t0 + c < ws.n_tiles) {
+                const uint16_t* r = recs + (size_t)(t0 + c) * kSfxStride;
+                const uint32_t ge = __ldcg(r + lo1), g2 = __ldcg(r + lo1 + 1);
+                gt[c] = (uint32_t)__ldcg(r + 257) + g2;
+                eq[c] = ge - g2;
+            }
+            sum_gt += gt[c];
+            sum_eq += eq[c];
         }
-        uint32_t igt = gt, ieq = eq;  // inclusive warp scans
+        if (p0 == 0) __threadfence();  // row_meta is visible before any prefix (= readiness) is
+        uint32_t igt = sum_gt, ieq = sum_eq;  // inclusive warp scans
 #pragma unroll
         for (int off = 1; off < 32; off <<= 1) {
             const uint32_t a = __shfl_up_sync(0xFFFFFFFFu, igt, off);
@@ -235,7 +212,7 @@ __device__ __forceinline__ void scan_row(SelectSmem& sm, int row, int n_kept, co
             sm.wsum[1][warp] = ieq;
         }
         __syncthreads();
-        uint32_t pg = carry_gt, pe = carry_eq, tg = 0, te = 0;
+        uint32_t pg = carry_gt + igt - sum_gt, pe = carry_eq + ieq - sum_eq, tg = 0, te = 0;
 #pragma unroll
         for (int w = 0; w < 8; ++w) {
             pg += (w < warp) ? sm.wsum[0][w] : 0u;
@@ -243,11 +220,15 @@ __device__ __forceinline__ void scan_row(SelectSmem& sm, int row, int n_kept, co
             tg += sm.wsum[0][w];
             te += sm.wsum[1][w];
         }
-        if (t < ws.n_tiles) {
-            const uint2 val = make_uint2(pg + igt - gt + 1u, pe + ieq - eq + 1u);  // +1: 0 means not ready
-            // 8-byte store: both halves become visible together
-            *reinterpret_cast<volatile unsigned long long*>(prefix + t) =
-                (unsigned long long)val.x | ((unsigned long long)val.y << 32);
+#pragma unroll
+        for (int c = 0; c < kScanTiles; ++c) {
+            if (t0 + c < ws.n_tiles) {
+                // 8-byte store: both halves become visible together; +1: 0 means not ready
+                *reinterpret_cast<volatile unsigned long long*>(prefix + t0 + c) =
+                    (unsigned long long)(pg + 1u) | ((unsigned long long)(pe + 1u) << 32);
+            }
+            pg += gt[c];
+            pe += eq[c];
         }
         carry_gt += tg;
         carry_eq += te;
@@ -337,10 +318,15 @@ __device__ __forceinline__ void refine_item(SelectSmem& sm, int row, int group, 
         }
         __syncwarp();
     }
-    // warp's share of the row's low-byte histogram
+    // the CTA's share of the row's low-byte histogram: warps summed in shared memory first, then one coalesced atomic
+    // per bin (per-warp atomics put 8 x 32 scattered sector updates per warp on the row's 256 counters)
 #pragma unroll
-    for (int i = 0; i < 8; ++i)
-        if (acc[i]) atomicAdd(&ws.hist_lo[(size_t)row * 256 + lane * 8 + i], acc[i]);
+    for (int i = 0; i < 8; ++i) lo[lane * 8 + i] = acc[i];
+    __syncthreads();
+    uint32_t bin_sum = 0;
+#pragma unroll
+    for (int w = 0; w < kTileThreads / 32; ++w) bin_sum += sm.lo[w][tid];
+    if (bin_sum) atomicAdd(&ws.hist_lo[(size_t)row * 256 + tid], bin_sum);
     __threadfence();
     __syncthreads();
     if (tid == 0) sm.last = (atomicAdd(&ws.counters[1 + row], 1u) == (uint32_t)(n_groups - 1));
@@ -351,70 +337,26 @@ __device__ __forceinline__ void refine_item(SelectSmem& sm, int row, int group, 
     }
 }
 
-// ---- compact item: (row, tile of kTile == kTileThreads positions, one per thread) ---------------------
-// kKeysReady: the row's keys were complete before this kernel started (two-kernel path): their load is issued BEFORE
-// the wait for the row scan, and the polling thread fetches the row's threshold right behind the flag, so an item is
-// ticket -> (keys || flag + threshold) -> rank -> copy instead of five dependent global round trips (ncu: CTA-barrier
-// waits behind those round trips were the top stall of this kernel, profiles/r02_prof_ea_select_details.txt).
-template <typename TR = void, bool kKeysReady = false>  // TR = void: plain copy; TR = cache dtype: KeyRerotationPress epilogue
-__device__ __forceinline__ void compact_item(SelectSmem& sm, int row, int tile, const char* K,
-                                             const char* V, Strides3 ks, Strides3 vs, char* K_out,
-                                             char* V_out, int32_t* idx_out, int H, int S, int D,
-                                             int n_kept, const Workspace& ws,
-                                             const float* inv_freq = nullptr) {
+// ---- rank + copy of one (row, tile of kTile == kTileThreads positions, one per thread) ------------------
+// key: this thread's position's ordered key; T / n_take: the row's threshold key and ties to take (row scan);
+// gt_before / eq_before: kept (> T) and tied (== T) positions in the row's tiles before this one.
+// Shared by the compaction grid and the fused Knorm kernel's compact items.
+template <typename TR, int U>  // TR = void: plain copy; TR = cache dtype: KeyRerotationPress epilogue
+__device__ __forceinline__ void rank_and_copy(int* list, uint32_t (&wsum)[2][8], int row, int tile, uint32_t key,
+                                              uint32_t T, uint32_t n_take, uint32_t gt_before, uint32_t eq_before,
+                                              const char* K, const char* V, Strides3 ks, Strides3 vs, char* K_out,
+                                              char* V_out, int32_t* idx_out, int H, int S, int D, int n_kept,
+                                              const float* inv_freq) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int b = row / H, h = row % H;
     const int s = tile * kTile + tid;
-    uint32_t key = 0;
-    if (kKeysReady) key = __ldcg(&ws.keys[(size_t)row * ws.S_pad + s]);  // in flight during the wait below
-    SEL_T0(t_wait);
-    // The row scan publishes tile_prefix[row][tile] = {kept_before + 1, tied_before + 1} last (the table is
-    // zeroed by the per-call memset), so one polled load doubles as the readiness flag (bounded spin;
-    // traps instead of hanging the GPU).
-    if (tid == 0) {
-        const volatile unsigned long long* slot =
-            reinterpret_cast<const volatile unsigned long long*>(ws.tile_prefix + (size_t)row * ws.n_tiles + tile);
-        volatile uint32_t* err = ws.counters + kCounterErrSlot(ws.R);
-        uint32_t spins = 0;
-        unsigned long long raw = *slot;
-        sm.abort = 0;
-        while ((uint32_t)raw == 0u || (uint32_t)(raw >> 32) == 0u) {
-            __nanosleep(64);
-            if (++spins > kSpinLimit) *err = 1u;          // raise: the host reports it, nobody traps
-            if ((spins & 255u) == 0u && *err != 0u) {     // raised here or by another CTA: drain
-                sm.abort = 1;
-                break;
-            }
-            raw = *slot;
-        }
-        const uint2 v = make_uint2((uint32_t)raw, (uint32_t)(raw >> 32));
-        __threadfence();
-        sm.thr[0] = v.x - 1u;
-        sm.thr[1] = v.y - 1u;
-        if (!sm.abort) {  // published before the prefix table (scan_row): valid once the flag is up
-            const uint2 m = __ldcg(&ws.row_meta[row]);
-            sm.meta[0] = m.x;
-            sm.meta[1] = m.y;
-        }
-    }
-    __syncthreads();
-    if (sm.abort) return;
-    SEL_ACC(0, t_wait);
-    SEL_T0(t_rank);
-    if (!kKeysReady) key = __ldcg(&ws.keys[(size_t)row * ws.S_pad + s]);
-    const uint2 meta = make_uint2(sm.meta[0], sm.meta[1]);
-    const uint2 before = make_uint2(sm.thr[0], sm.thr[1]);
-    const uint32_t T = meta.x, n_take = meta.y;
-    const uint32_t gt_before = before.x, eq_before = before.y;
-
     const bool valid = s < S;
     const bool is_gt = valid && key > T;
     const bool is_eq = valid && key == T;
     const unsigned m_gt = __ballot_sync(0xFFFFFFFFu, is_gt);
     const unsigned m_eq = __ballot_sync(0xFFFFFFFFu, is_eq);
     if (lane == 0) {
-        sm.wsum[0][warp] = __popc(m_gt);
-        sm.wsum[1][warp] = __popc(m_eq);
+        wsum[0][warp] = __popc(m_gt);
+        wsum[1][warp] = __popc(m_eq);
     }
     __syncthreads();
     uint32_t gt_rank = __popc(m_gt & ((1u << lane) - 1u));
@@ -422,93 +364,72 @@ __device__ __forceinline__ void compact_item(SelectSmem& sm, int row, int tile, 
     uint32_t tot_gt = 0, tot_eq = 0;
 #pragma unroll
     for (int w = 0; w < 8; ++w) {
-        gt_rank += (w < warp) ? sm.wsum[0][w] : 0u;
-        eq_rank += (w < warp) ? sm.wsum[1][w] : 0u;
-        tot_gt += sm.wsum[0][w];
-        tot_eq += sm.wsum[1][w];
+        gt_rank += (w < warp) ? wsum[0][w] : 0u;
+        eq_rank += (w < warp) ? wsum[1][w] : 0u;
+        tot_gt += wsum[0][w];
+        tot_eq += wsum[1][w];
     }
     // ties are taken in position order: this tile may take those with global tie rank < n_take
     const uint32_t tie_room = (n_take > eq_before) ? (n_take - eq_before) : 0u;
     const uint32_t out_base = gt_before + min(eq_before, n_take);
-    if (is_gt || (is_eq && eq_rank < tie_room)) sm.list[gt_rank + min(eq_rank, tie_room)] = s;
+    if (is_gt || (is_eq && eq_rank < tie_room)) list[gt_rank + min(eq_rank, tie_room)] = s;
     const int count = (int)(tot_gt + min(tot_eq, tie_room));
     __syncthreads();
-    SEL_ACC(1, t_rank);
-    SEL_T0(t_copy);
-    if (count > 0) {
-        const int64_t out_row0 = (int64_t)row * n_kept + out_base;
-        if (idx_out != nullptr && tid < count) idx_out[out_row0 + tid] = sm.list[tid];
-        const int64_t row_bytes = (int64_t)D * 2;
-        const char* k_src = K + ((int64_t)b * ks.b + (int64_t)h * ks.h) * 2;
-        const char* v_src = V + ((int64_t)b * vs.b + (int64_t)h * vs.h) * 2;
-        if (K_out == nullptr) {
-            // selection only (kvp_scores_select): the kept positions in idx_out are the whole result
-        } else if constexpr (std::is_void<TR>::value) {
-            copy_rows_kv<KVP_SEL_U, KVP_SEL_TWO>(k_src, ks.s * 2, v_src, vs.s * 2, K_out + out_row0 * row_bytes,
-                                                 V_out + out_row0 * row_bytes, row_bytes, sm.list, count, D >> 3);
-        } else {
-            copy_rows_k_rerotated<TR>(k_src, ks.s * 2, K_out + out_row0 * row_bytes, row_bytes, sm.list, count, D,
-                                      inv_freq, (int)out_base);
-            copy_rows_single(v_src, vs.s * 2, V_out + out_row0 * row_bytes, row_bytes, sm.list, count, D >> 3);
-        }
+    if (count == 0) return;
+    const int b = row / H, h = row % H;
+    const int64_t out_row0 = (int64_t)row * n_kept + out_base;
+    if (idx_out != nullptr && tid < count) idx_out[out_row0 + tid] = list[tid];
+    const int64_t row_bytes = (int64_t)D * 2;
+    const char* k_src = K + ((int64_t)b * ks.b + (int64_t)h * ks.h) * 2;
+    const char* v_src = V + ((int64_t)b * vs.b + (int64_t)h * vs.h) * 2;
+    if (K_out == nullptr) {
+        // selection only (kvp_scores_select): the kept positions in idx_out are the whole result
+    } else if constexpr (std::is_void<TR>::value) {
+        copy_rows_kv<U>(k_src, ks.s * 2, v_src, vs.s * 2, K_out + out_row0 * row_bytes, V_out + out_row0 * row_bytes,
+                        row_bytes, list, count, D >> 3);
+    } else {
+        copy_rows_k_rerotated<TR>(k_src, ks.s * 2, K_out + out_row0 * row_bytes, row_bytes, list, count, D, inv_freq,
+                                  (int)out_base);
+        copy_rows_single(v_src, vs.s * 2, V_out + out_row0 * row_bytes, row_bytes, list, count, D >> 3);
     }
-    SEL_ACC(2, t_copy);
-    SEL_CNT(3);
 }
 
-// Persistent select+compact kernel: CTAs pull items from one ticket counter. Items [0, nA) are the
-// refine items (the last one to finish for a row also runs that row's scan and raises its ready
-// flag), items [nA, nA + nB) the compact items (last rows / last tiles first, so K rows the score
-// stage touched last are re-read while still in L2). A compact item only waits for refine items,
-// which precede it in the queue and never wait themselves => no deadlock for any grid size.
-#ifndef KVP_REROT_CTAS
-#define KVP_REROT_CTAS 4  // re-rotating variant: 64 regs, 4 CTAs/SM (issue-bound on sincosf; A/B 220 -> 207 us, profiles/r01_ab_rerot.txt)
-#endif
-template <typename TR>
-__global__ void __launch_bounds__(kTileThreads, std::is_void<TR>::value ? KVP_SEL_CTAS : KVP_REROT_CTAS)
-select_compact_kernel(const char* __restrict__ K, const char* __restrict__ V, Strides3 ks,
-                      Strides3 vs, char* __restrict__ K_out, char* __restrict__ V_out,
-                      int32_t* __restrict__ idx_out, int H, int S, int D, int n_kept,
-                      Workspace ws, const float* __restrict__ inv_freq) {
+// ---- selection pass: one CTA per refine item (row, group of kGroupTiles tiles) ----------------------------
+// Nothing here waits on another CTA, so a plain grid of any size is safe. The CTA that completes a row's last
+// item runs that row's scan. Dependents are released at once: the compaction grid can take residency while
+// this pass runs and parks in its pdl_wait() until the pass has completed.
+__global__ void __launch_bounds__(kTileThreads)
+select_kernel(int S, int n_kept, Workspace ws) {
     __shared__ SelectSmem sm;
-    const int R = ws.R;
-    const int n_groups = (ws.n_tiles + kGroupTiles - 1) / kGroupTiles;
-    const int nA = R * n_groups, nB = R * ws.n_tiles;
+    pdl_launch_dependents();
     pdl_wait();  // keys + histograms of the score stage are complete and visible
-    SEL_T0(t_kernel);
-    // The ticket of the NEXT item is drawn while the current one is processed (its round trip hides behind the item).
-    // A CTA therefore holds one ticket it has not started; deadlock-free as before: a held refine ticket belongs to a
-    // CTA that is processing an earlier refine item, and refine items never wait.
-    uint32_t next_ticket = 0;
-    if (threadIdx.x == 0) next_ticket = atomicAdd(&ws.counters[0], 1u);
-    while (true) {
-        SEL_T0(t_ticket);
-        __syncthreads();  // previous item's shared state is dead
-        if (threadIdx.x == 0) sm.item = (int)next_ticket;
-        __syncthreads();
-        SEL_ACC(4, t_ticket);
-        const int item = sm.item;
-        if (item >= nA + nB) break;
-        if (threadIdx.x == 0) next_ticket = atomicAdd(&ws.counters[0], 1u);
-        if (item < nA) {
-            SEL_T0(t_ref);
-            refine_item(sm, item / n_groups, item % n_groups, n_groups, S, n_kept, ws);
-            SEL_ACC(5, t_ref);
-            SEL_CNT(6);
-        } else {
-            const int j = item - nA;
-            const int row = R - 1 - j / ws.n_tiles;
-            const int tile = ws.n_tiles - 1 - j % ws.n_tiles;
-            compact_item<TR, true>(sm, row, tile, K, V, ks, vs, K_out, V_out, idx_out, H, S, D, n_kept, ws, inv_freq);
-        }
-    }
-    SEL_ACC(7, t_kernel);
+    const int n_groups = (ws.n_tiles + kGroupTiles - 1) / kGroupTiles;
+    refine_item(sm, blockIdx.x / n_groups, blockIdx.x % n_groups, n_groups, S, n_kept, ws);
 }
 
-template <typename Kern>
-static int persistent_grid(Kern kernel, int threads, int n_items, PerDeviceInt& occupancy) {
-    const int grid = device_sm_count() * cached_ctas_per_sm(kernel, threads, occupancy);
-    return n_items < grid ? n_items : grid;
+// ---- compaction grid: one CTA per (row, tile), last rows / last tiles first ---------------------------------
+// 1-D grid (gridDim.y would cap the row count at 65535). After pdl_wait() the keys, the tile prefix and the row's
+// threshold are final, so the three loads are independent and the CTA never waits for another one.
+// Register budget (ptxas -v, sm_100a): no spills at the bound below; A/B of the (U, CTAs/SM) settings in DESIGN.md §4.1.
+constexpr int kCompactU = 2;
+constexpr int kCompactCtas = 4;
+constexpr int kRerotCtas = 4;  // re-rotating variant: issue-bound on sincosf (A/B 220 -> 207 us, profiles/r01_ab_rerot.txt)
+template <typename TR>
+__global__ void __launch_bounds__(kTileThreads, std::is_void<TR>::value ? kCompactCtas : kRerotCtas)
+compact_kernel(const char* __restrict__ K, const char* __restrict__ V, Strides3 ks, Strides3 vs,
+               char* __restrict__ K_out, char* __restrict__ V_out, int32_t* __restrict__ idx_out, int H, int S, int D,
+               int n_kept, Workspace ws, const float* __restrict__ inv_freq) {
+    __shared__ int list[kTile];
+    __shared__ uint32_t wsum[2][8];
+    const int n_tiles = ws.n_tiles;
+    const int row = ws.R - 1 - (int)(blockIdx.x / (unsigned)n_tiles);
+    const int tile = n_tiles - 1 - (int)(blockIdx.x % (unsigned)n_tiles);
+    pdl_wait();  // the selection pass (and through it the score stage) has completed
+    const uint32_t key = __ldcg(&ws.keys[(size_t)row * ws.S_pad + (size_t)tile * kTile + threadIdx.x]);
+    const uint2 before = __ldcg(&ws.tile_prefix[(size_t)row * n_tiles + tile]);  // +1 encoded (scan_row)
+    const uint2 meta = __ldcg(&ws.row_meta[row]);
+    rank_and_copy<TR, kCompactU>(list, wsum, row, tile, key, meta.x, meta.y, before.x - 1u, before.y - 1u, K, V, ks,
+                                 vs, K_out, V_out, idx_out, H, S, D, n_kept, inv_freq);
 }
 
 template <typename TR>
@@ -516,18 +437,19 @@ static cudaError_t launch_select_compact_t(const Dims& d, const void* K, const v
                                            void* V_out, int32_t* idx_out, const Workspace& ws,
                                            const float* inv_freq, cudaStream_t st) {
     const int n_groups = (ws.n_tiles + kGroupTiles - 1) / kGroupTiles;
-    const int n_items = d.R * n_groups + d.R * ws.n_tiles;
-    auto kern = select_compact_kernel<TR>;
-    static PerDeviceInt occupancy;  // one per <TR> instantiation of this launcher
-    const int grid = persistent_grid(kern, kTileThreads, n_items, occupancy);
+    const dim3 sel_grid(d.R * n_groups), cmp_grid(d.R * ws.n_tiles);
+    auto cmp = compact_kernel<TR>;
 #ifndef KVP_NO_PDL
-    return launch_pdl(kern, dim3(grid), dim3(kTileThreads), 0, st, static_cast<const char*>(K),
+    cudaError_t e = launch_pdl(select_kernel, sel_grid, dim3(kTileThreads), 0, st, d.S, d.n_kept, ws);
+    if (e != cudaSuccess) return e;
+    return launch_pdl(cmp, cmp_grid, dim3(kTileThreads), 0, st, static_cast<const char*>(K),
                       static_cast<const char*>(V), d.ks, d.vs, static_cast<char*>(K_out), static_cast<char*>(V_out),
                       idx_out, d.H, d.S, d.D, d.n_kept, ws, inv_freq);
 #else
-    kern<<<grid, kTileThreads, 0, st>>>(static_cast<const char*>(K), static_cast<const char*>(V), d.ks, d.vs,
-                                        static_cast<char*>(K_out), static_cast<char*>(V_out), idx_out, d.H,
-                                        d.S, d.D, d.n_kept, ws, inv_freq);
+    select_kernel<<<sel_grid, kTileThreads, 0, st>>>(d.S, d.n_kept, ws);
+    cmp<<<cmp_grid, kTileThreads, 0, st>>>(static_cast<const char*>(K), static_cast<const char*>(V), d.ks, d.vs,
+                                           static_cast<char*>(K_out), static_cast<char*>(V_out), idx_out, d.H, d.S,
+                                           d.D, d.n_kept, ws, inv_freq);
     return cudaPeekAtLastError();
 #endif
 }
@@ -635,6 +557,52 @@ __device__ __forceinline__ bool spin_until(const uint32_t* counter, uint32_t nee
     return true;
 }
 
+// Compact item of the fused queue: (row, tile) polls its tile prefix, which the row scan publishes last (the table
+// is zeroed by the per-call memset, so one polled load doubles as the readiness flag; bounded spin), and the polling
+// thread fetches the row's threshold right behind it. The keys are loaded after the wait: the score items of the
+// same launch write them.
+__device__ __forceinline__ void fused_compact_item(SelectSmem& sm, int row, int tile, const char* K, const char* V,
+                                                   Strides3 ks, Strides3 vs, char* K_out, char* V_out,
+                                                   int32_t* idx_out, int H, int S, int D, int n_kept,
+                                                   const Workspace& ws) {
+    if (threadIdx.x == 0) {
+        const volatile unsigned long long* slot =
+            reinterpret_cast<const volatile unsigned long long*>(ws.tile_prefix + (size_t)row * ws.n_tiles + tile);
+        volatile uint32_t* err = ws.counters + kCounterErrSlot(ws.R);
+        uint32_t spins = 0;
+        unsigned long long raw = *slot;
+        sm.abort = 0;
+        while ((uint32_t)raw == 0u || (uint32_t)(raw >> 32) == 0u) {
+            __nanosleep(64);
+            if (++spins > kSpinLimit) *err = 1u;          // raise: the host reports it, nobody traps
+            if ((spins & 255u) == 0u && *err != 0u) {     // raised here or by another CTA: drain
+                sm.abort = 1;
+                break;
+            }
+            raw = *slot;
+        }
+        __threadfence();
+        sm.thr[0] = (uint32_t)raw - 1u;
+        sm.thr[1] = (uint32_t)(raw >> 32) - 1u;
+        if (!sm.abort) {  // published before the prefix table (scan_row): valid once the flag is up
+            const uint2 m = __ldcg(&ws.row_meta[row]);
+            sm.meta[0] = m.x;
+            sm.meta[1] = m.y;
+        }
+    }
+    __syncthreads();
+    if (sm.abort) return;
+    const uint32_t key = __ldcg(&ws.keys[(size_t)row * ws.S_pad + (size_t)tile * kTile + threadIdx.x]);
+    rank_and_copy<void, 3>(sm.list, sm.wsum, row, tile, key, sm.meta[0], sm.meta[1], sm.thr[0], sm.thr[1], K, V, ks,
+                           vs, K_out, V_out, idx_out, H, S, D, n_kept, nullptr);
+}
+
+template <typename Kern>
+static int persistent_grid(Kern kernel, int threads, int n_items, PerDeviceInt& occupancy) {
+    const int grid = device_sm_count() * cached_ctas_per_sm(kernel, threads, occupancy);
+    return n_items < grid ? n_items : grid;
+}
+
 template <typename T, int LPR>
 __global__ void __launch_bounds__(kTileThreads, 3)
 knorm_fused_kernel(const T* __restrict__ K, const T* __restrict__ V, Strides3 ks, Strides3 vs,
@@ -674,9 +642,9 @@ knorm_fused_kernel(const T* __restrict__ K, const T* __restrict__ V, Strides3 ks
             if (sm.abort) continue;
             refine_item(sm, it.row, it.idx, nA, S, n_kept, ws);
         } else {
-            compact_item(sm, it.row, it.idx, reinterpret_cast<const char*>(K),
-                         reinterpret_cast<const char*>(V), ks, vs, K_out, V_out, idx_out, H, S, D, n_kept,
-                         ws);
+            fused_compact_item(sm, it.row, it.idx, reinterpret_cast<const char*>(K),
+                               reinterpret_cast<const char*>(V), ks, vs, K_out, V_out, idx_out, H, S, D, n_kept,
+                               ws);
         }
     }
 }
@@ -759,10 +727,10 @@ streaming_compact_kernel(const char* __restrict__ K, const char* __restrict__ V,
     if (idx_out != nullptr)
         for (int j = tid; j < count; j += kTileThreads) idx_out[out_row0 + j] = s_list[j];
     const int64_t row_bytes = (int64_t)D * 2;
-    copy_rows_kv<4, true>(K + ((int64_t)b * ks.b + (int64_t)h * ks.h) * 2, ks.s * 2,
-                 V + ((int64_t)b * vs.b + (int64_t)h * vs.h) * 2, vs.s * 2,
-                 K_out + out_row0 * row_bytes, V_out + out_row0 * row_bytes, row_bytes, s_list, count,
-                 D >> 3);
+    copy_rows_kv<4>(K + ((int64_t)b * ks.b + (int64_t)h * ks.h) * 2, ks.s * 2,
+                    V + ((int64_t)b * vs.b + (int64_t)h * vs.h) * 2, vs.s * 2,
+                    K_out + out_row0 * row_bytes, V_out + out_row0 * row_bytes, row_bytes, s_list, count,
+                    D >> 3);
 }
 
 cudaError_t launch_streaming_compress(const Dims& d, int n_sink, const void* K, const void* V,

@@ -535,7 +535,7 @@ snap_finalize_kernel(int S, int window, int kernel_size, float inv_gw, SnapScrat
     __shared__ float s_max[8];
     const int tile = blockIdx.x, row = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     shist[tid] = 0;
-    pdl_launch_dependents();  // the select+compact kernel behind this one may start to take residency
+    pdl_launch_dependents();  // the selection pass behind this one may start to take residency
     const int n_scored = S - window;
     float fmax_valid = -INFINITY;
     for (int sub = 0; sub < kFinalizeTiles; ++sub) {

@@ -282,7 +282,7 @@ class GraphedCall:
 
     The C-ABI calls only enqueue kernels / memset nodes on the current stream (the ExpectedAttention side
     stream forks from and joins back into it), never synchronise and never allocate, so they are capturable
-    as they are. `replay()` costs one cudaGraphLaunch on the host instead of 1-6 launches + their argument
+    as they are. `replay()` costs one cudaGraphLaunch on the host instead of 1-7 launches + their argument
     marshalling: it makes the call GPU-bound on any host (DecodingPress compactions, repeated same-shape
     prefill layers, bench.py). Outputs are the tensors `fn` returned; they are overwritten by every replay.
     The inputs must stay alive and at the same addresses (update them in place)."""
